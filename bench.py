@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py -- headline benchmark of the wlseg hot path (contract: see the task statement).
+"""bench.py -- headline benchmark of the wlseg hot path.
 
 BASELINE.json's metric has two halves; the default run measures BOTH in one process and prints ONE line:
 
@@ -15,8 +15,11 @@ BASELINE.json's metric has two halves; the default run measures BOTH in one proc
   python bench.py --impl reference --steps K --warmup W  # the reference algorithm on the host CPU (oracle port;
                                                          # TF 1.12 is uninstallable): the training step, same
                                                          # config as the headline, eval nested
+  python bench.py --dump-outputs DIR ...                 # also write what the last timed step computed, as
+                                                         # DIR/<name>.npy, so that two builds can be compared
 
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  The inputs and the initial parameters are seeded: the same arguments give the same
+inputs on every run.
 """
 
 import argparse
@@ -55,7 +58,14 @@ def parse_args():
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-e2e', action='store_true')
   ap.add_argument('--detail', type=str, default=None, help='write the per-kernel-class roofline table here')
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', type=str, default=None, metavar='DIR',
+                  help='write the outputs of the last timed step as DIR/<name>.npy (float32 / float64)')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'wlseg':
+    ap.error('--dump-outputs records the wlseg arm only')
+  return args
 
 
 def load_peaks():
@@ -87,6 +97,17 @@ def load_traffic(workload, kernel_prefix):
   if not n:
     return None, None
   return sum(v['dram_bytes_per_launch'] * v['launches'] for v in hits) / n, files[-1]
+
+
+def dump_outputs(out_dir, arrays):
+  """--dump-outputs: every array as out_dir/<name>.npy, integer and float64 arrays as float64 (exact for counts below
+  2**53), the others as float32."""
+  import numpy as np
+  import torch
+  os.makedirs(out_dir, exist_ok=True)
+  for name, t in arrays.items():
+    t = t.detach().double() if t.dtype in (torch.int32, torch.int64, torch.float64) else t.detach().float()
+    np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
 
 
 class ClockSampler:
@@ -266,19 +287,17 @@ def reference_train_record(args, steps, warm):
 
 def run_reference(args):
   """Reference arm: the reference's own algorithm (oracle port) on the host cores, rank 0 only.  Same config as the
-  GPU arm (a full per-GPU batch per step); the step COUNT is bounded so that the run ends within a few minutes
-  (a 4 x 768 x 768 fp32 training step takes ~10 s on 16 cores, a 4 x 1024 x 2048 evaluation step ~10 s)."""
+  GPU arm (a full per-GPU batch per step) and the same step counts: a 4 x 768 x 768 fp32 training step takes ~10 s on
+  16 cores, a 4 x 1024 x 2048 evaluation step ~10 s, so pass a small --steps / --warmup here."""
   rank = int(os.environ.get('RANK', '0'))
   if rank != 0:
     return
-  steps = max(1, min(args.steps, 4))
-  warm = max(0, min(args.warmup, 1))
   if args.workload == 'eval':
-    line = reference_eval_record(args, steps, warm)
+    line = reference_eval_record(args, args.steps, args.warmup)
   else:
-    line = reference_train_record(args, steps, warm)
+    line = reference_train_record(args, args.steps, args.warmup)
     if args.workload == 'both':
-      line['eval'] = reference_eval_record(args, max(1, min(args.steps, 2)), warm)
+      line['eval'] = reference_eval_record(args, args.steps, args.warmup)
   print(json.dumps(line), flush=True)
 
 
@@ -399,6 +418,10 @@ def run_wlseg_eval(args, ctx):
   clocks = sampler.stop() if sampler else None
   ms = e0.elapsed_time(e1)
   assert int(cm.sum()) == world * args.steps * NB * H * W, 'confusion matrix does not cover the timed pixels'
+  if args.dump_outputs and rank == 0:
+    # what a caller of the evaluation step receives: the confusion matrix over the timed steps (it was reset before
+    # them) and the count of labels outside the class range
+    dump_outputs(args.dump_outputs, {'eval_confusion_matrix': cm, 'eval_invalid_labels': evstep.invalid})
   t = torch.tensor([ms], dtype=torch.float64, device=dev)
   if world > 1:
     dist.all_reduce(t, op=dist.ReduceOp.MAX)

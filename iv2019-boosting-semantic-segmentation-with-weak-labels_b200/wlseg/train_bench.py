@@ -65,6 +65,12 @@ def run(args, ctx, cpu_train_sample=None):
   torch.cuda.synchronize()
   clocks = sampler.stop() if sampler else None
   ms = e0.elapsed_time(e1)
+  if args.dump_outputs and rank == 0:
+    # what a caller of the training step receives: the loss vector of the last timed step.  The updated parameters are
+    # left out: from random init this network amplifies rounding-order differences ~10^2 per step (DESIGN.md), and
+    # after the default 3 + 20 steps two runs of one build hold momentum slots with cosine ~0 (measured on a B200 at
+    # 1000 W), while their losses agree to 1e-2 relative
+    bench.dump_outputs(args.dump_outputs, {'train_losses': out})
   # roofline pass, live, right after the timed region: the same steps launched eagerly with a CUDA
   # event pair around every convolution launch (events cannot sit inside a replayed graph)
   prof_steps = min(3, args.steps)
