@@ -439,6 +439,28 @@ int wlseg_resize_crop(const void* x, void* y, int32_t N, int32_t H, int32_t W, i
                       int32_t RW, int32_t oy, int32_t ox, int32_t TH, int32_t TW, int32_t kind,
                       wlseg_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Evaluation inputs from raw bytes (the EVAL contract of SURVEY.md 3.5 as the reference's
+ * evaluation pipeline produces it, with the arithmetic of _predict_preprocess,
+ * input_pipelines/dataset_agnostic/dataset_agnostic_predict_input.py:109-119), for a batch whose
+ * examples each have their own size:
+ *   images    uint8 [N, cap_img]: row n holds an RGB image packed HWC, H_n x W_n x 3 bytes
+ *   lids      uint8 [N, cap_lab]: row n holds its label-id map, H_n x W_n bytes
+ *   sizes     int32 [N, 2] = (H_n, W_n)
+ *   lut       int32 [n_lids], n_lids <= 256: label id -> class id (_replacevoids(lids2cids))
+ *   proimages fp32  [N, TH, TW, 3] = (bilinear(u8 * (float)(1/255)) - 0.5) / 0.5, TF-1.12 legacy
+ *             bilinear (align_corners=False), every operation rounded separately (bit-equal to
+ *             wlseg/image_input.py)
+ *   prolabels int32 [N, TH, TW] = lut[nearest(lids)], legacy nearest (align_corners=False)
+ *   *invalid  int64, accumulated into (the caller zeroes): + 1 per label id >= n_lids (that pixel
+ *             gets void_id) and + 1 per example whose size does not fit cap_img / cap_lab (its
+ *             outputs are not written).
+ * ------------------------------------------------------------------------------------------ */
+int wlseg_eval_inputs(const uint8_t* images, int64_t cap_img, const uint8_t* lids, int64_t cap_lab,
+                      const int32_t* sizes, int32_t N, const int32_t* lut, int32_t n_lids, int32_t void_id,
+                      int32_t TH, int32_t TW, float* proimages, int32_t* prolabels, int64_t* invalid,
+                      wlseg_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

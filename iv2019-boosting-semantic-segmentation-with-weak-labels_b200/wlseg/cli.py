@@ -67,7 +67,16 @@ def evaluate_main(argv):
   ss = wsettings.build_parser(wsettings.EVAL)
   st = wsettings.eval_extra_args(ss.parse_args(argv))
   _dist_env(st)
-  system = SemanticSegmentation({'eval': synthetic.eval_input_fn}, None, st)
+  # real images from the split directory tfrecords_path names unless --synthetic or it is no split in a known layout
+  from wlseg import dataset_input
+  layout = None if getattr(st, 'synthetic', False) else dataset_input.detect_layout(st.tfrecords_path)
+  if layout:
+    print(f'Evaluating the {layout} split at {st.tfrecords_path}.')
+  else:
+    why = ('--synthetic is given' if getattr(st, 'synthetic', False) else
+           f'{st.tfrecords_path} is not a Cityscapes leftImg8bit/<split> or Vistas split (images/ + labels/) directory')
+    print(f'Evaluating SYNTHETIC input: {why}.')
+  system = SemanticSegmentation({'eval': dataset_input.eval_input_fn if layout else synthetic.eval_input_fn}, None, st)
   labels = system.settings.evaluation_problem_def['cids2labels']
   void_exists = -1 in system.settings.evaluation_problem_def['lids2cids']
   if void_exists and not system.settings.train_void_class:

@@ -14,6 +14,7 @@ import numpy as np
 import torch
 
 from wlseg import checkpoints, network, ops
+from wlseg.dataset_input import PACKED_IMAGES, PACKED_LIDS, PACKED_SIZES
 
 
 def _replacevoids(mappings):
@@ -269,7 +270,8 @@ class Estimator:
   # ---- EVAL ---------------------------------------------------------------------------------------
   def evaluate(self, batches, num_classes, lut=None):
     """define_estimator EVAL branch: forward, remap cids, resize to label size, streaming confusion
-    matrix.  `batches` yields (features, labels) with host or device tensors.  Returns the
+    matrix.  `batches` yields (features, labels) with host or device tensors, as proimages / prolabels or in the
+    packed raw form of wlseg.dataset_input (converted on the device by `_raw_eval_inputs`).  Returns the
     reference's metrics dict {'confusion_matrix': np.int32[C, C], 'loss': 0.0, 'global_step'}."""
     dev = self.device
     lut_t = None if lut is None else torch.tensor(lut, dtype=torch.int32, device=dev)
@@ -288,7 +290,12 @@ class Estimator:
     host_cm = self.__dict__.setdefault('_host_cm', {}).get(num_classes)
     if host_cm is None:   # pinned once: cudaHostAlloc per call costs more than a step's worth of launches
       host_cm = self._host_cm[num_classes] = torch.zeros((num_classes, num_classes), dtype=torch.int64).pin_memory()
+    raw = None
     for features, labels in pre:
+      if PACKED_IMAGES in features:
+        if raw is None:
+          raw = self._raw_eval_inputs()
+        features, labels = raw(features, labels)
       lab = labels['prolabels']
       if tuple(lab.shape[1:3]) == tuple(features['proimages'].shape[1:3]) and self.params.upsampling != 'no':
         step(features['proimages'], lab)
@@ -305,12 +312,39 @@ class Estimator:
     torch.cuda.synchronize(dev)
     self.last_h2d_bytes = pre.h2d_bytes
     self.last_d2h_bytes = steps * host_cm.numel() * 8
+    if raw is not None and int(raw.invalid.item()):
+      raise ops.WlsegError(f'{int(raw.invalid.item())} label ids outside the evaluation problem definition\'s lids2cids '
+                           'table, or examples larger than their batch rows')
     if int(invalid.item()):
       raise ops.WlsegError(f'{int(invalid.item())} (label, decision) pairs outside [0, {num_classes})')
     total = cm.cpu().numpy()
     # the reference exposes tf.to_int32(total_cm)
     return {'confusion_matrix': total.astype(np.int32), 'confusion_matrix_int64': total, 'loss': 0.0,
             'global_step': self.global_step, 'steps': steps}
+
+  def _raw_eval_inputs(self):
+    """Converter of batches in packed raw form (wlseg.dataset_input) into the evaluation contract on the device
+    (ops.eval_inputs).  Results go to one estimator-owned (proimages, prolabels) pair per (N, TH, TW), so EvalStep sees
+    recurring addresses and replays its graph without copying.  The label-id table of the evaluation problem definition
+    is uploaded once per call; `.invalid` counts what the kernel rejected."""
+    s = self.settings
+    table = _replacevoids(s.evaluation_problem_def['lids2cids'])
+    lut = torch.tensor(table, dtype=torch.int32, device=self.device)
+    th, tw = s.height_feature_extractor, s.width_feature_extractor
+    outs = self.__dict__.setdefault('_raw_eval_outputs', {})
+    invalid = torch.zeros(1, dtype=torch.int64, device=self.device)
+
+    def convert(features, labels):
+      images = features[PACKED_IMAGES]
+      key = (images.shape[0], th, tw)
+      if key not in outs:
+        outs[key] = (torch.empty(key + (3,), dtype=torch.float32, device=self.device),
+                     torch.empty(key, dtype=torch.int32, device=self.device))
+      pro, lab = outs[key]
+      ops.eval_inputs(images, labels[PACKED_LIDS], features[PACKED_SIZES], lut, max(table), (th, tw), pro, lab, invalid)
+      return {'proimages': pro}, {'prolabels': lab}
+    convert.invalid = invalid
+    return convert
 
   # ---- PREDICT ------------------------------------------------------------------------------------
   def predict(self, batches, predict_keys):

@@ -109,6 +109,8 @@ _SIGNATURES = {
     'wlseg_zero_insert': (ctypes.c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int, _vp]),
     'wlseg_conv1_pack': (ctypes.c_int, [_vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp]),
     'wlseg_resize_crop': (ctypes.c_int, [_vp, _vp] + [_c_int] * 11 + [_vp]),
+    'wlseg_eval_inputs': (ctypes.c_int, [_vp, _c_i64, _vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _c_int, _vp,
+                                         _vp, _vp, _vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
@@ -624,3 +626,24 @@ def resize_crop(x, resized_hw, offset, target_hw, kind):
          'wlseg_resize_crop')
   _count()
   return y.squeeze(-1) if squeeze else y
+
+
+def eval_inputs(images, lids, sizes, lut, void_id, target_hw, proimages, prolabels, invalid):
+  """Raw examples of their own sizes -> the evaluation contract, one launch (wlseg_eval_inputs).  images uint8
+  [N, cap_img] (RGB packed HWC per row), lids uint8 [N, cap_lab], sizes int32 [N, 2] = (H, W), lut int32 [<= 256]
+  label id -> class id.  Writes proimages fp32 [N, TH, TW, 3] and prolabels int32 [N, TH, TW]; invalid (int64 [1]) +=
+  the out-of-range label ids and the examples whose size does not fit their row."""
+  N = images.shape[0]
+  TH, TW = int(target_hw[0]), int(target_hw[1])
+  assert images.dtype == torch.uint8 and lids.dtype == torch.uint8 and images.dim() == 2 and lids.dim() == 2
+  assert images.is_contiguous() and lids.is_contiguous() and lids.shape[0] == N
+  assert sizes.dtype == torch.int32 and sizes.is_contiguous() and tuple(sizes.shape) == (N, 2)
+  assert lut.dtype == torch.int32 and lut.is_contiguous() and lut.dim() == 1
+  assert proimages.dtype == torch.float32 and proimages.is_contiguous() and tuple(proimages.shape) == (N, TH, TW, 3)
+  assert prolabels.dtype == torch.int32 and prolabels.is_contiguous() and tuple(prolabels.shape) == (N, TH, TW)
+  assert invalid.dtype == torch.int64
+  _check(lib().wlseg_eval_inputs(_ptr(images), images.shape[1], _ptr(lids), lids.shape[1], _ptr(sizes), N, _ptr(lut),
+                                 lut.numel(), int(void_id), TH, TW, _ptr(proimages), _ptr(prolabels), _ptr(invalid),
+                                 _stream()), 'wlseg_eval_inputs')
+  _count()
+  return proimages, prolabels
