@@ -461,6 +461,25 @@ int wlseg_eval_inputs(const uint8_t* images, int64_t cap_img, const uint8_t* lid
                       int32_t TH, int32_t TW, float* proimages, int32_t* prolabels, int64_t* invalid,
                       wlseg_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Training inputs (the per-pixel part of the TRAIN contract of SURVEY.md 3.5) gathered from a
+ * device-resident arena of raw examples.  train.py does not preserve the aspect ratio of per-pixel
+ * examples, so a training example is exactly the per-pixel arithmetic of wlseg_eval_inputs (one
+ * shared device function):
+ *   arena      uint8, ragged: example e starts at byte offsets[e] (int64: arenas exceed 4 GiB) with
+ *              its RGB image packed HWC (H_e x W_e x 3 bytes), then its label-id map (H_e x W_e)
+ *   sizes      int32 [n_examples, 2] = (H_e, W_e)
+ *   index      int32 [N], device memory: output example n is arena example index[n]
+ *   lut, void_id, TH, TW, proimages, prolabels: as wlseg_eval_inputs
+ *   *invalid   int64, accumulated into (the caller zeroes): + 1 per label id >= n_lids (that pixel
+ *              gets void_id) and + 1 per index outside [0, n_examples) or example of non-positive
+ *              size (its outputs are not written).
+ * ------------------------------------------------------------------------------------------ */
+int wlseg_train_inputs(const uint8_t* arena, const int64_t* offsets, const int32_t* sizes, int32_t n_examples,
+                       const int32_t* index, int32_t N, const int32_t* lut, int32_t n_lids, int32_t void_id,
+                       int32_t TH, int32_t TW, float* proimages, int32_t* prolabels, int64_t* invalid,
+                       wlseg_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -40,15 +40,49 @@ resize_crop_kernel(const T* __restrict__ x, T* __restrict__ y, int N, int H, int
   }
 }
 
-// Evaluation input contract (SURVEY.md 3.5) from raw bytes, one thread per output pixel.  Example n is an RGB image
-// packed HWC at its own size sizes[n] = (H, W) in row n of `images` (cap_img bytes per row) and its label-id map in
-// row n of `lids` (cap_lab bytes per row).
+// Per-pixel input contract (SURVEY.md 3.5) of output pixel (Y, X) from one raw example: an RGB image packed HWC at
+// H x W and its label-id map.  Shared by the evaluation and training kernels, so that their bit equality with the host
+// pipeline lives in one place.
 //   image: u8 -> float * (float)(1/255) (tf.image.convert_image_dtype multiplies), TF-1.12 legacy bilinear
 //          (align_corners=False, x first, then y), (v - 0.5) / 0.5.  Every operation is rounded on its own
 //          (__f*_rn keep the compiler from contracting the lerps into FMAs): the host pipeline of wlseg/image_input.py
 //          and oracle/preprocess.py round that way, and the contract is bit equality with them.
-//   labels: legacy nearest, then lut[id] from shared memory; an id >= n_lids writes void_id and is counted.
-// A row whose size does not fit its buffers writes nothing and counts once.
+//   labels: legacy nearest, then lut[id] from shared memory; an id >= n_lids writes void_id and returns false.
+__device__ __forceinline__ bool input_contract_pixel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ lids,
+                                                     int H, int W, int Y, int X, int TH, int TW,
+                                                     const int32_t* s_lut, int n_lids, int void_id,
+                                                     float* __restrict__ pro, int32_t* __restrict__ lab) {
+  const float inv255 = 1.0f / 255.0f;
+  // [TF-1.12] CalculateResizeScale without align_corners: in / static_cast<float>(out)
+  const float sy = __fdiv_rn((float)H, (float)TH), sx = __fdiv_rn((float)W, (float)TW);
+  const float fy = __fmul_rn((float)Y, sy), fx = __fmul_rn((float)X, sx);
+  const float fly = floorf(fy), flx = floorf(fx);
+  const int yl = min((int)fly, H - 1), xl = min((int)flx, W - 1);
+  const int yh = min(yl + 1, H - 1), xh = min(xl + 1, W - 1);
+  const float ly = __fsub_rn(fy, fly), lx = __fsub_rn(fx, flx);
+  const uint8_t* ptl = img + ((int64_t)yl * W + xl) * 3;
+  const uint8_t* ptr = img + ((int64_t)yl * W + xh) * 3;
+  const uint8_t* pbl = img + ((int64_t)yh * W + xl) * 3;
+  const uint8_t* pbr = img + ((int64_t)yh * W + xh) * 3;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float tl = __fmul_rn((float)__ldg(ptl + c), inv255), tr = __fmul_rn((float)__ldg(ptr + c), inv255);
+    const float bl = __fmul_rn((float)__ldg(pbl + c), inv255), br = __fmul_rn((float)__ldg(pbr + c), inv255);
+    const float top = __fadd_rn(tl, __fmul_rn(__fsub_rn(tr, tl), lx));
+    const float bot = __fadd_rn(bl, __fmul_rn(__fsub_rn(br, bl), lx));
+    const float v = __fadd_rn(top, __fmul_rn(__fsub_rn(bot, top), ly));
+    pro[c] = __fmul_rn(__fsub_rn(v, 0.5f), 2.0f);   // / 0.5 is exact as * 2
+  }
+  const int id = __ldg(lids + (int64_t)yl * W + xl);   // nearest: the same min(floor(.), in - 1)
+  const bool ok = id < n_lids;
+  *lab = ok ? s_lut[id] : void_id;
+  return ok;
+}
+
+// Evaluation input contract from raw bytes, one thread per output pixel.  Example n is an RGB image packed HWC at its
+// own size sizes[n] = (H, W) in row n of `images` (cap_img bytes per row) and its label-id map in row n of `lids`
+// (cap_lab bytes per row).  A row whose size does not fit its buffers writes nothing and counts once; an out-of-range
+// label id counts once per output pixel.
 __global__ void __launch_bounds__(256)
 eval_inputs_kernel(const uint8_t* __restrict__ images, int64_t cap_img, const uint8_t* __restrict__ lids, int64_t cap_lab,
                    const int32_t* __restrict__ sizes, int N, const int32_t* __restrict__ lut, int n_lids, int void_id,
@@ -57,7 +91,6 @@ eval_inputs_kernel(const uint8_t* __restrict__ images, int64_t cap_img, const ui
   __shared__ int32_t s_lut[256];
   for (int i = threadIdx.x; i < n_lids; i += blockDim.x) s_lut[i] = lut[i];
   __syncthreads();
-  const float inv255 = 1.0f / 255.0f;
   unsigned bad = 0;
   const int64_t total = (int64_t)N * TH * TW;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -70,33 +103,48 @@ eval_inputs_kernel(const uint8_t* __restrict__ images, int64_t cap_img, const ui
       bad += (X == 0 && Y == 0);
       continue;
     }
-    // [TF-1.12] CalculateResizeScale without align_corners: in / static_cast<float>(out)
-    const float sy = __fdiv_rn((float)H, (float)TH), sx = __fdiv_rn((float)W, (float)TW);
-    const float fy = __fmul_rn((float)Y, sy), fx = __fmul_rn((float)X, sx);
-    const float fly = floorf(fy), flx = floorf(fx);
-    const int yl = min((int)fly, H - 1), xl = min((int)flx, W - 1);
-    const int yh = min(yl + 1, H - 1), xh = min(xl + 1, W - 1);
-    const float ly = __fsub_rn(fy, fly), lx = __fsub_rn(fx, flx);
-    const uint8_t* img = images + (int64_t)n * cap_img;
-    const uint8_t* ptl = img + ((int64_t)yl * W + xl) * 3;
-    const uint8_t* ptr = img + ((int64_t)yl * W + xh) * 3;
-    const uint8_t* pbl = img + ((int64_t)yh * W + xl) * 3;
-    const uint8_t* pbr = img + ((int64_t)yh * W + xh) * 3;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      const float tl = __fmul_rn((float)__ldg(ptl + c), inv255), tr = __fmul_rn((float)__ldg(ptr + c), inv255);
-      const float bl = __fmul_rn((float)__ldg(pbl + c), inv255), br = __fmul_rn((float)__ldg(pbr + c), inv255);
-      const float top = __fadd_rn(tl, __fmul_rn(__fsub_rn(tr, tl), lx));
-      const float bot = __fadd_rn(bl, __fmul_rn(__fsub_rn(br, bl), lx));
-      const float v = __fadd_rn(top, __fmul_rn(__fsub_rn(bot, top), ly));
-      pro[i * 3 + c] = __fmul_rn(__fsub_rn(v, 0.5f), 2.0f);   // / 0.5 is exact as * 2
-    }
-    const int id = __ldg(lids + (int64_t)n * cap_lab + (int64_t)yl * W + xl);   // nearest: the same min(floor(.), in - 1)
-    const bool ok = id < n_lids;
-    bad += !ok;
-    lab[i] = ok ? s_lut[id] : void_id;
+    bad += !input_contract_pixel(images + (int64_t)n * cap_img, lids + (int64_t)n * cap_lab, H, W, Y, X, TH, TW, s_lut,
+                                 n_lids, void_id, pro + i * 3, lab + i);
   }
   // one atomic per warp: every lane leaves the grid-stride loop before this point
+  const unsigned warp_bad = __reduce_add_sync(0xffffffffu, bad);
+  if ((threadIdx.x & 31) == 0 && warp_bad) atomicAdd(invalid, (unsigned long long)warp_bad);
+}
+
+// Training input contract (per-pixel part of the batch) gathered from a device-resident arena of raw examples, one
+// thread per output pixel.  Output example n is arena example e = index[n]: its RGB image (H x W x 3 bytes, HWC) starts
+// at byte offsets[e] and its label-id map (H x W bytes) follows it; sizes[e] = (H, W).  An index outside
+// [0, n_examples) or a non-positive size writes nothing for that example and counts once; an out-of-range label id
+// counts once per output pixel.
+__global__ void __launch_bounds__(256)
+train_inputs_kernel(const uint8_t* __restrict__ arena, const int64_t* __restrict__ offsets,
+                    const int32_t* __restrict__ sizes, int n_examples, const int32_t* __restrict__ index, int N,
+                    const int32_t* __restrict__ lut, int n_lids, int void_id, int TH, int TW, float* __restrict__ pro,
+                    int32_t* __restrict__ lab, unsigned long long* __restrict__ invalid) {
+  __shared__ int32_t s_lut[256];
+  for (int i = threadIdx.x; i < n_lids; i += blockDim.x) s_lut[i] = lut[i];
+  __syncthreads();
+  unsigned bad = 0;
+  const int64_t total = (int64_t)N * TH * TW;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int X = (int)(i % TW);
+    const int64_t t = i / TW;
+    const int Y = (int)(t % TH);
+    const int n = (int)(t / TH);
+    const int e = __ldg(index + n);
+    if (e < 0 || e >= n_examples) {
+      bad += (X == 0 && Y == 0);
+      continue;
+    }
+    const int H = __ldg(sizes + 2 * e), W = __ldg(sizes + 2 * e + 1);
+    if (H <= 0 || W <= 0) {
+      bad += (X == 0 && Y == 0);
+      continue;
+    }
+    const uint8_t* img = arena + __ldg(offsets + e);
+    bad += !input_contract_pixel(img, img + (int64_t)H * W * 3, H, W, Y, X, TH, TW, s_lut, n_lids, void_id, pro + i * 3,
+                                 lab + i);
+  }
   const unsigned warp_bad = __reduce_add_sync(0xffffffffu, bad);
   if ((threadIdx.x & 31) == 0 && warp_bad) atomicAdd(invalid, (unsigned long long)warp_bad);
 }
@@ -136,6 +184,23 @@ extern "C" int wlseg_eval_inputs(const uint8_t* images, int64_t cap_img, const u
   const int grid = bw_grid((int64_t)N * TH * TW, 256, 8);
   eval_inputs_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(images, cap_img, lids, cap_lab, sizes, N, lut, n_lids, void_id,
                                                              TH, TW, proimages, prolabels, (unsigned long long*)invalid);
+  WLSEG_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int wlseg_train_inputs(const uint8_t* arena, const int64_t* offsets, const int32_t* sizes, int32_t n_examples,
+                                  const int32_t* index, int32_t N, const int32_t* lut, int32_t n_lids, int32_t void_id,
+                                  int32_t TH, int32_t TW, float* proimages, int32_t* prolabels, int64_t* invalid,
+                                  wlseg_stream_t stream) {
+  WLSEG_CHECK_ARG(N >= 0 && n_examples >= 0 && TH > 0 && TW > 0, "train_inputs: bad geometry");
+  WLSEG_CHECK_ARG(n_lids >= 1 && n_lids <= 256, "train_inputs: the label-id table has %d entries, 1..256 supported", n_lids);
+  if (N == 0) return 0;
+  WLSEG_CHECK_ARG(index && lut && proimages && prolabels && invalid, "train_inputs: null pointer");
+  WLSEG_CHECK_ARG(n_examples == 0 || (arena && offsets && sizes), "train_inputs: null arena");
+  const int grid = bw_grid((int64_t)N * TH * TW, 256, 8);
+  train_inputs_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(arena, offsets, sizes, n_examples, index, N, lut, n_lids,
+                                                              void_id, TH, TW, proimages, prolabels,
+                                                              (unsigned long long*)invalid);
   WLSEG_LAUNCH_CHECK();
   return 0;
 }

@@ -56,7 +56,15 @@ def train_main(argv):
     # 0's would be saved.  The reference is one process for all GPUs and needs the flag to use more than one.
     raise ValueError(f'WORLD_SIZE={st.world_size} but --distribute is not set: launch one process, or pass --distribute '
                      'for data-parallel training.')
-  system = SemanticSegmentation({'train': synthetic.train_input_fn}, None, st)
+  input_fn = synthetic.train_input_fn
+  if st.per_pixel_split_path and not st.synthetic:
+    from wlseg import train_input
+    pairs = train_input.split_pairs(st.per_pixel_split_path, st.per_pixel_dataset_name)
+    print(f'Training on the {st.per_pixel_dataset_name} split at {st.per_pixel_split_path}: {len(pairs)} image / label '
+          f'pairs, {len(pairs[st.rank::st.world_size])} on this rank; the bounding-box and image-level parts of the batch '
+          'are empty (there is no Open Images source).', flush=True)
+    input_fn = train_input.train_input_fn
+  system = SemanticSegmentation({'train': input_fn}, None, st)
   out = system.train()
   _dist_shutdown(st, system)
   return out

@@ -214,6 +214,9 @@ class Estimator:
         variables, _ = checkpoints.load_file(init)
         mapping = checkpoints.warm_start(self.params, variables, psp_module=getattr(self.settings, 'psp_module', False))
         print(f'initialised {len(mapping)} variables from {init}', flush=True)
+    if for_training:
+      # the step training continues from: an input function that follows a data order (wlseg.train_input) resumes there
+      self.settings.initial_global_step = self.global_step
     self.__dict__.pop('_eval_steps', None)   # graphs captured for a previous network object
     # group norm has no folded inference form: its evaluation forward is the training forward (network.py)
     cls = network.TrainNetwork if self.params.norm == 'group' else network.Network

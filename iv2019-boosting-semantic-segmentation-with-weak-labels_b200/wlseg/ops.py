@@ -111,6 +111,8 @@ _SIGNATURES = {
     'wlseg_resize_crop': (ctypes.c_int, [_vp, _vp] + [_c_int] * 11 + [_vp]),
     'wlseg_eval_inputs': (ctypes.c_int, [_vp, _c_i64, _vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _c_int, _vp,
                                          _vp, _vp, _vp]),
+    'wlseg_train_inputs': (ctypes.c_int, [_vp, _vp, _vp, _c_int, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp,
+                                          _vp, _vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
@@ -645,5 +647,28 @@ def eval_inputs(images, lids, sizes, lut, void_id, target_hw, proimages, prolabe
   _check(lib().wlseg_eval_inputs(_ptr(images), images.shape[1], _ptr(lids), lids.shape[1], _ptr(sizes), N, _ptr(lut),
                                  lut.numel(), int(void_id), TH, TW, _ptr(proimages), _ptr(prolabels), _ptr(invalid),
                                  _stream()), 'wlseg_eval_inputs')
+  _count()
+  return proimages, prolabels
+
+
+def train_inputs(arena, offsets, sizes, index, lut, void_id, target_hw, proimages, prolabels, invalid):
+  """Arena examples selected by a device index vector -> the per-pixel training contract, one launch
+  (wlseg_train_inputs).  arena uint8 [bytes] (example e at offsets[e]: RGB HWC, then its label-id map), offsets int64
+  [E], sizes int32 [E, 2] = (H, W), index int32 [N], lut int32 [<= 256] label id -> class id.  Writes proimages fp32
+  [N, TH, TW, 3] and prolabels int32 [N, TH, TW]; invalid (int64 [1]) += the out-of-range label ids and indices."""
+  N = index.numel()
+  E = offsets.numel()
+  TH, TW = int(target_hw[0]), int(target_hw[1])
+  assert arena.dtype == torch.uint8 and arena.dim() == 1 and arena.is_contiguous()
+  assert offsets.dtype == torch.int64 and offsets.is_contiguous() and offsets.dim() == 1
+  assert sizes.dtype == torch.int32 and sizes.is_contiguous() and tuple(sizes.shape) == (E, 2)
+  assert index.dtype == torch.int32 and index.is_contiguous() and index.dim() == 1
+  assert lut.dtype == torch.int32 and lut.is_contiguous() and lut.dim() == 1
+  assert proimages.dtype == torch.float32 and proimages.is_contiguous() and tuple(proimages.shape) == (N, TH, TW, 3)
+  assert prolabels.dtype == torch.int32 and prolabels.is_contiguous() and tuple(prolabels.shape) == (N, TH, TW)
+  assert invalid.dtype == torch.int64
+  _check(lib().wlseg_train_inputs(_ptr(arena), _ptr(offsets), _ptr(sizes), E, _ptr(index), N, _ptr(lut), lut.numel(),
+                                  int(void_id), TH, TW, _ptr(proimages), _ptr(prolabels), _ptr(invalid), _stream()),
+         'wlseg_train_inputs')
   _count()
   return proimages, prolabels

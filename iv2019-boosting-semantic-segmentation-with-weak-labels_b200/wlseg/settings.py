@@ -7,7 +7,8 @@ code/input_pipelines/dataset_agnostic/dataset_agnostic_predict_input.py:156-164)
 flags (code/predict.py:171-197) and the per-script hard overrides (`_add_extra_args`:
 code/train.py:42-68, code/evaluate.py:69-79, code/predict.py:199-211).
 
-Additive flags of this implementation (absent upstream): --synthetic, --dtype, --steps, --seed.
+Additive flags of this implementation (absent upstream): --synthetic, --dtype, --steps, --seed, and for train.py
+--per_pixel_split_path.
 """
 
 import argparse
@@ -20,6 +21,7 @@ class SemanticSegmentationArguments(object):
 
   def __init__(self, mode=None):
     self._parser = argparse.ArgumentParser()
+    self._mode = mode
     self.add_system_arguments()
     self.add_tf_arguments()
     if mode == PREDICT:
@@ -57,6 +59,10 @@ class SemanticSegmentationArguments(object):
                    help='bf16: tcgen05 product path; fp32: check mode (direct fp32 convolutions).')
     p.add_argument('--steps', type=int, default=None, help='Stop after this many steps.')
     p.add_argument('--seed', type=int, default=0)
+    if self._mode == TRAIN:
+      p.add_argument('--per_pixel_split_path', type=str, default=None, metavar='DIR',
+                     help='Training split of the per-pixel dataset (a Cityscapes leftImg8bit/<split> directory or a Vistas '
+                          'split directory with images/ + labels/), decoded once into device memory.')
 
   def add_train_arguments(self):
     p = self._parser
