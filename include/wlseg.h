@@ -480,6 +480,36 @@ int wlseg_train_inputs(const uint8_t* arena, const int64_t* offsets, const int32
                        int32_t TH, int32_t TW, float* proimages, int32_t* prolabels, int64_t* invalid,
                        wlseg_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Training inputs of one weak part of the batch (the bounding-box or the image-level examples
+ * of the TRAIN contract of SURVEY.md 3.5) gathered from a device-resident arena of RGB images.
+ * train.py preserves the aspect ratio of weak examples: example e (H x W) is resized to
+ * resized[e] = (RH, RW) = wlseg.preprocess.resized_size(H, W, (TH, TW), True) and cropped to
+ * TH x TW at the per-output offset crops[n] = (oy, ox).
+ *   arena      uint8: example e is H_e x W_e x 3 bytes (RGB, HWC) at byte offsets[e] (int64)
+ *   sizes, resized  int32 [n_examples, 2]
+ *   box_start  int32 [n_examples + 1] or NULL: boxes [box_start[e], box_start[e + 1]) of example e
+ *              in box_coords (fp32 [boxes, 4] = xmin, xmax, ymin, ymax normalised, 16-byte
+ *              aligned) and box_cids (int32 [boxes], weak class id; ids outside 0..14 are skipped)
+ *   vectors    fp32 [n_examples, 15] or NULL: one image-level multinomial per example.  Exactly one
+ *              of box_start and vectors is given.
+ *   index      int32 [N], crops int32 [N, 2]: output example n is arena example index[n] cut at
+ *              crops[n]; N <= 65535
+ *   proimages  fp32 [N, TH, TW, 3]: the image arithmetic of wlseg_train_inputs at the resized size
+ *              (u8 / 255, legacy bilinear, [-1, 1)), sampled at (Y + oy, X + ox)
+ *   labels     fp32 [N, TH, TW, 15]: bbox part = _generate_rla at H x W, then legacy nearest to
+ *              RH x RW, then the crop (bit-equal to wlseg_rasterize_bbox_labels + wlseg_resize_crop);
+ *              image-level part = vectors[index[n]] at every pixel
+ *   *invalid   int64, accumulated into (the caller zeroes): + 1 per output example whose index is
+ *              outside [0, n_examples), whose crop is outside [0, RH - TH] x [0, RW - TW], whose
+ *              size is not positive or that has more than 1024 boxes (its outputs are not written).
+ * ------------------------------------------------------------------------------------------ */
+int wlseg_weak_train_inputs(const uint8_t* arena, const int64_t* offsets, const int32_t* sizes,
+                            const int32_t* resized, int32_t n_examples, const int32_t* box_start,
+                            const float* box_coords, const int32_t* box_cids, const float* vectors,
+                            const int32_t* index, const int32_t* crops, int32_t N, int32_t TH, int32_t TW,
+                            float* proimages, float* labels, int64_t* invalid, wlseg_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

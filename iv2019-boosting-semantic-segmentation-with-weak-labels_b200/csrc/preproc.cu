@@ -6,7 +6,7 @@
 //   window of the target size is cut out of them.
 // One pass: the crop window is read straight out of the source - the resized full-size tensor never exists.
 // Bandwidth kernel, one thread per output element (consecutive threads = consecutive addresses).
-#include "common.cuh"
+#include "weak_boxes.cuh"
 
 namespace wlseg {
 
@@ -40,22 +40,23 @@ resize_crop_kernel(const T* __restrict__ x, T* __restrict__ y, int N, int H, int
   }
 }
 
-// Per-pixel input contract (SURVEY.md 3.5) of output pixel (Y, X) from one raw example: an RGB image packed HWC at
-// H x W and its label-id map.  Shared by the evaluation and training kernels, so that their bit equality with the host
-// pipeline lives in one place.
-//   image: u8 -> float * (float)(1/255) (tf.image.convert_image_dtype multiplies), TF-1.12 legacy bilinear
-//          (align_corners=False, x first, then y), (v - 0.5) / 0.5.  Every operation is rounded on its own
-//          (__f*_rn keep the compiler from contracting the lerps into FMAs): the host pipeline of wlseg/image_input.py
-//          and oracle/preprocess.py round that way, and the contract is bit equality with them.
-//   labels: legacy nearest, then lut[id] from shared memory; an id >= n_lids writes void_id and returns false.
-__device__ __forceinline__ bool input_contract_pixel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ lids,
-                                                     int H, int W, int Y, int X, int TH, int TW,
-                                                     const int32_t* s_lut, int n_lids, int void_id,
-                                                     float* __restrict__ pro, int32_t* __restrict__ lab) {
+// [TF-1.12] CalculateResizeScale without align_corners: in / static_cast<float>(out)
+__device__ __forceinline__ float legacy_scale(int in, int out) { return __fdiv_rn((float)in, (float)out); }
+
+// Image part of the input contract (SURVEY.md 3.5) at one output pixel: an RGB image packed HWC at H x W, resized with
+// the scales sy = legacy_scale(H, RH), sx = legacy_scale(W, RW) and sampled at (Ys, Xs) of the resized grid (the crop
+// window's offset is already added).
+//   u8 -> float * (float)(1/255) (tf.image.convert_image_dtype multiplies), TF-1.12 legacy bilinear (align_corners=False,
+//   x first, then y), (v - 0.5) / 0.5.  Every operation is rounded on its own (__f*_rn keep the compiler from
+//   contracting the lerps into FMAs): the host pipeline of wlseg/image_input.py and oracle/preprocess.py round that way,
+//   and the contract is bit equality with them.
+// -> the nearest source pixel (yl, xl) = min(floor(.), in - 1), which is also where legacy nearest reads labels.
+struct SrcPixel { int y, x; };
+
+__device__ __forceinline__ SrcPixel contract_image_pixel(const uint8_t* __restrict__ img, int H, int W, float sy, float sx,
+                                                     int Ys, int Xs, float* __restrict__ pro) {
   const float inv255 = 1.0f / 255.0f;
-  // [TF-1.12] CalculateResizeScale without align_corners: in / static_cast<float>(out)
-  const float sy = __fdiv_rn((float)H, (float)TH), sx = __fdiv_rn((float)W, (float)TW);
-  const float fy = __fmul_rn((float)Y, sy), fx = __fmul_rn((float)X, sx);
+  const float fy = __fmul_rn((float)Ys, sy), fx = __fmul_rn((float)Xs, sx);
   const float fly = floorf(fy), flx = floorf(fx);
   const int yl = min((int)fly, H - 1), xl = min((int)flx, W - 1);
   const int yh = min(yl + 1, H - 1), xh = min(xl + 1, W - 1);
@@ -73,7 +74,19 @@ __device__ __forceinline__ bool input_contract_pixel(const uint8_t* __restrict__
     const float v = __fadd_rn(top, __fmul_rn(__fsub_rn(bot, top), ly));
     pro[c] = __fmul_rn(__fsub_rn(v, 0.5f), 2.0f);   // / 0.5 is exact as * 2
   }
-  const int id = __ldg(lids + (int64_t)yl * W + xl);   // nearest: the same min(floor(.), in - 1)
+  return SrcPixel{yl, xl};
+}
+
+// Per-pixel input contract of output pixel (Y, X) from one raw example: the image part above resized straight to the
+// target size, and the label-id map with legacy nearest, then lut[id] from shared memory; an id >= n_lids writes
+// void_id and returns false.  Shared by the evaluation and training kernels, so that their bit equality with the host
+// pipeline lives in one place.
+__device__ __forceinline__ bool input_contract_pixel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ lids,
+                                                     int H, int W, int Y, int X, int TH, int TW,
+                                                     const int32_t* s_lut, int n_lids, int void_id,
+                                                     float* __restrict__ pro, int32_t* __restrict__ lab) {
+  const SrcPixel src = contract_image_pixel(img, H, W, legacy_scale(H, TH), legacy_scale(W, TW), Y, X, pro);
+  const int id = __ldg(lids + (int64_t)src.y * W + src.x);   // nearest: the same min(floor(.), in - 1)
   const bool ok = id < n_lids;
   *lab = ok ? s_lut[id] : void_id;
   return ok;
@@ -149,6 +162,97 @@ train_inputs_kernel(const uint8_t* __restrict__ arena, const int64_t* __restrict
   if ((threadIdx.x & 31) == 0 && warp_bad) atomicAdd(invalid, (unsigned long long)warp_bad);
 }
 
+// Weak part of the training batch (bounding-box or image-level examples, SURVEY.md 3.5) gathered from a
+// device-resident arena, one thread per output pixel and one row of CTAs (blockIdx.y) per output example.  Output
+// example n is arena example e = index[n]: an RGB image (H x W x 3 bytes, HWC) at byte offsets[e], resized (aspect
+// preserved) to resized[e] = (RH, RW) and cropped to TH x TW at crops[n] = (oy, ox).  Its label is, for the bbox part,
+// _generate_rla of the boxes [box_start[e], box_start[e + 1]) rasterised at H x W, read with legacy nearest at the
+// source pixel the image's bilinear lower corner uses; for the image-level part, vectors[e] at every pixel.  An index
+// outside [0, n_examples), a crop outside [0, RH - TH] x [0, RW - TW], a non-positive size or more than kMaxBoxesSmem
+// boxes writes nothing for that example and counts once.
+constexpr int kWeakThreads = 256;
+
+__global__ void __launch_bounds__(kWeakThreads)
+weak_train_inputs_kernel(const uint8_t* __restrict__ arena, const int64_t* __restrict__ offsets,
+                         const int32_t* __restrict__ sizes, const int32_t* __restrict__ resized, int n_examples,
+                         const int32_t* __restrict__ box_start, const float4* __restrict__ box_coords,
+                         const int32_t* __restrict__ box_cids, const float* __restrict__ vectors,
+                         const int32_t* __restrict__ index, const int32_t* __restrict__ crops, int TH, int TW,
+                         float* __restrict__ pro, float* __restrict__ lab, unsigned long long* __restrict__ invalid) {
+  __shared__ BoxI boxes[kMaxBoxesSmem];
+  __shared__ float s_vec[kWeakC];
+  __shared__ float s_scale[2];
+  __shared__ int nbox;
+  __shared__ float stage[kWeakThreads * kWeakC];
+  const int n = blockIdx.y;
+  const int e = __ldg(index + n);
+  // every thread of the CTA reaches the same verdict, so an invalid example leaves as a whole
+  bool ok = e >= 0 && e < n_examples;
+  int H = 0, W = 0, RH = 0, RW = 0, oy = 0, ox = 0, b0 = 0, b1 = 0;
+  if (ok) {
+    H = __ldg(sizes + 2 * e), W = __ldg(sizes + 2 * e + 1);
+    RH = __ldg(resized + 2 * e), RW = __ldg(resized + 2 * e + 1);
+    oy = __ldg(crops + 2 * n), ox = __ldg(crops + 2 * n + 1);
+    ok = H > 0 && W > 0 && oy >= 0 && ox >= 0 && oy <= RH - TH && ox <= RW - TW;
+    if (box_start != nullptr) {
+      b0 = __ldg(box_start + e), b1 = __ldg(box_start + e + 1);
+      ok = ok && b0 >= 0 && b1 >= b0 && b1 - b0 <= kMaxBoxesSmem;
+    }
+  }
+  if (!ok) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(invalid, 1ull);
+    return;
+  }
+  // the two scale divisions in different warps: one thread computing both keeps the first result across the second's
+  // slow-path call in local memory
+  if (threadIdx.x == 0) {
+    nbox = 0;
+    s_scale[0] = legacy_scale(H, RH);
+  }
+  if (threadIdx.x == 32) s_scale[1] = legacy_scale(W, RW);
+  if (vectors != nullptr && threadIdx.x < kWeakC) s_vec[threadIdx.x] = __ldg(vectors + (int64_t)e * kWeakC + threadIdx.x);
+  __syncthreads();
+  // integer corners at H x W of the example's boxes (cids outside [0, 14] are skipped, as the reference skips mids that
+  // are not in mid2cid); slots come in any order, the counts they add are order-free
+  for (int b = b0 + threadIdx.x; b < b1; b += kWeakThreads) {
+    const int cid = __ldg(box_cids + b);
+    if (cid < 0 || cid >= kWeakC) continue;
+    const float4 c = __ldg(box_coords + b);
+    BoxI bx;
+    if (box_corners(c.x, c.y, c.z, c.w, cid, H, W, bx)) boxes[atomicAdd(&nbox, 1)] = bx;   // b1 - b0 <= kMaxBoxesSmem
+  }
+  __syncthreads();
+  const uint8_t* img = arena + __ldg(offsets + e);
+  const int64_t npix = (int64_t)TH * TW;
+  float* pro_n = pro + (int64_t)n * npix * 3;
+  float* lab_n = lab + (int64_t)n * npix * kWeakC;
+  for (int64_t p0 = (int64_t)blockIdx.x * kWeakThreads; p0 < npix; p0 += (int64_t)gridDim.x * kWeakThreads) {
+    const int64_t p = p0 + threadIdx.x;
+    float v[kWeakC];
+    if (p < npix) {
+      const int Y = (int)p / TW, X = (int)p - Y * TW;   // TH * TW < 2^31 (checked at launch)
+      // the scales are read from shared memory per pixel: held in registers across the slow-path calls of the box
+      // divisions, one of them spills to local memory
+      const float sy = *(volatile float*)&s_scale[0], sx = *(volatile float*)&s_scale[1];
+      const SrcPixel src = contract_image_pixel(img, H, W, sy, sx, Y + oy, X + ox, pro_n + p * 3);
+      if (vectors != nullptr) {
+#pragma unroll
+        for (int c = 0; c < kWeakC; ++c) v[c] = s_vec[c];
+      } else {
+        box_multinomial(boxes, nbox, src.y, src.x, v);
+      }
+    }
+    // transpose through shared memory: the CTA's 256 x 15 floats are one contiguous span of the output
+    __syncthreads();
+#pragma unroll
+    for (int c = 0; c < kWeakC; ++c) stage[threadIdx.x * kWeakC + c] = v[c];
+    __syncthreads();
+    const int64_t valid = (npix - p0 < kWeakThreads ? npix - p0 : kWeakThreads) * kWeakC;
+    float* dst = lab_n + p0 * kWeakC;
+    for (int i = threadIdx.x; i < valid; i += kWeakThreads) dst[i] = stage[i];
+  }
+}
+
 }  // namespace wlseg
 
 using namespace wlseg;
@@ -201,6 +305,31 @@ extern "C" int wlseg_train_inputs(const uint8_t* arena, const int64_t* offsets, 
   train_inputs_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(arena, offsets, sizes, n_examples, index, N, lut, n_lids,
                                                               void_id, TH, TW, proimages, prolabels,
                                                               (unsigned long long*)invalid);
+  WLSEG_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int wlseg_weak_train_inputs(const uint8_t* arena, const int64_t* offsets, const int32_t* sizes,
+                                       const int32_t* resized, int32_t n_examples, const int32_t* box_start,
+                                       const float* box_coords, const int32_t* box_cids, const float* vectors,
+                                       const int32_t* index, const int32_t* crops, int32_t N, int32_t TH, int32_t TW,
+                                       float* proimages, float* labels, int64_t* invalid, wlseg_stream_t stream) {
+  WLSEG_CHECK_ARG(N >= 0 && N <= 65535 && n_examples >= 0 && TH > 0 && TW > 0 && (int64_t)TH * TW < (1ll << 31),
+                  "weak_train_inputs: bad geometry");
+  WLSEG_CHECK_ARG((box_start != nullptr) != (vectors != nullptr),
+                  "weak_train_inputs: give either the box table (bounding-box part) or the vectors (image-level part)");
+  if (N == 0) return 0;
+  WLSEG_CHECK_ARG(index && crops && proimages && labels && invalid, "weak_train_inputs: null pointer");
+  WLSEG_CHECK_ARG(n_examples == 0 || (arena && offsets && sizes && resized), "weak_train_inputs: null arena");
+  WLSEG_CHECK_ARG(box_start == nullptr || (box_coords && box_cids), "weak_train_inputs: null box table");
+  WLSEG_CHECK_ARG(((uintptr_t)box_coords & 15) == 0, "weak_train_inputs: box_coords must be 16-byte aligned");
+  const int64_t npix = (int64_t)TH * TW;
+  int gx = (int)ceil_div(npix, kWeakThreads);
+  const int cap = (kNumSMs * 8 + N - 1) / N;
+  if (gx > cap) gx = cap;
+  weak_train_inputs_kernel<<<dim3(gx, N), kWeakThreads, 0, (cudaStream_t)stream>>>(
+      arena, offsets, sizes, resized, n_examples, box_start, (const float4*)box_coords, box_cids, vectors, index, crops,
+      TH, TW, proimages, labels, (unsigned long long*)invalid);
   WLSEG_LAUNCH_CHECK();
   return 0;
 }

@@ -4,22 +4,16 @@
 //       overlapping boxes add counts, per-pixel normalisation to a multinomial, void where no box)
 //   code/input_pipelines/open_images/input_subset_image_labels.py:73-107 (uniform over the image's
 //       classes, tiled over the image)
-// Bit-exact with the numpy originals: box corners are int(coord * size) evaluated in double as numpy does
-// for float32 * int32, the slice [min : max + 1] is clipped to the image, counts are small integers and
-// the normalisation is one IEEE float32 division per channel.
+// The box arithmetic (bit-exact with the numpy original) is weak_boxes.cuh, shared with the training gather.
 //
 // Bandwidth kernel: writes 60 B per pixel, reads the <= a few hundred boxes of the image from shared
 // memory.  One thread per pixel; a CTA's 256 x 15 floats are one contiguous span of the output and leave
 // through a shared-memory transpose as fully coalesced stores.
-#include "common.cuh"
+#include "weak_boxes.cuh"
 
 namespace wlseg {
 
-constexpr int kWeakC = 15;          // 14 Open Images classes + void (input_subset_bboxes_v2.py:38-53)
 constexpr int kRastThreads = 256;
-constexpr int kMaxBoxesSmem = 1024;
-
-struct BoxI { int x0, x1, y0, y1, cid; };
 
 __global__ void __launch_bounds__(kRastThreads)
 rasterize_bbox_kernel(const float* __restrict__ coords, const int32_t* __restrict__ cids, int max_boxes, int H, int W,
@@ -37,18 +31,7 @@ rasterize_bbox_kernel(const float* __restrict__ coords, const int32_t* __restric
     if (cid < 0 || cid >= kWeakC) continue;
     const float* c = coords + ((int64_t)n * max_boxes + b) * 4;   // xmin, xmax, ymin, ymax (normalised)
     BoxI bx;
-    bx.x0 = (int)((double)c[0] * (double)W);
-    bx.x1 = (int)((double)c[1] * (double)W);
-    bx.y0 = (int)((double)c[2] * (double)H);
-    bx.y1 = (int)((double)c[3] * (double)H);
-    bx.cid = cid;
-    // python slice rla[y0 : y1 + 1, x0 : x1 + 1] for non-negative corners: clipped to the image,
-    // empty when min > max
-    if (bx.x0 < 0) bx.x0 = 0;
-    if (bx.y0 < 0) bx.y0 = 0;
-    if (bx.x1 > W - 1) bx.x1 = W - 1;
-    if (bx.y1 > H - 1) bx.y1 = H - 1;
-    if (bx.x0 > bx.x1 || bx.y0 > bx.y1) continue;
+    if (!box_corners(c[0], c[1], c[2], c[3], cid, H, W, bx)) continue;
     const int slot = atomicAdd(&nbox, 1);
     if (slot < kMaxBoxesSmem) boxes[slot] = bx;
   }
@@ -58,27 +41,7 @@ rasterize_bbox_kernel(const float* __restrict__ coords, const int32_t* __restric
   for (int64_t p0 = (int64_t)blockIdx.x * kRastThreads; p0 < npix; p0 += (int64_t)gridDim.x * kRastThreads) {
     const int64_t p = p0 + threadIdx.x;
     float v[kWeakC];
-#pragma unroll
-    for (int c = 0; c < kWeakC; ++c) v[c] = 0.f;
-    if (p < npix) {
-      const int y = (int)(p / W), x = (int)(p % W);
-      for (int b = 0; b < nb; ++b) {
-        const BoxI bx = boxes[b];
-        const bool in = (x >= bx.x0) & (x <= bx.x1) & (y >= bx.y0) & (y <= bx.y1);
-#pragma unroll
-        for (int c = 0; c < kWeakC; ++c) v[c] += (in && bx.cid == c) ? 1.f : 0.f;   // small integers: order-free
-      }
-      float s = 0.f;
-#pragma unroll
-      for (int c = 0; c < kWeakC; ++c) s += v[c];
-      if (s > 0.5f) {
-#pragma unroll
-        for (int c = 0; c < kWeakC; ++c) v[c] = __fdiv_rn(v[c], s);
-      } else {
-#pragma unroll
-        for (int c = 0; c < kWeakC; ++c) v[c] = (c == kWeakC - 1) ? 1.f : 0.f;
-      }
-    }
+    if (p < npix) box_multinomial(boxes, nb, (int)(p / W), (int)(p % W), v);
     // transpose through shared memory: the block's 256 x 15 floats are one contiguous span of the output
     __syncthreads();
 #pragma unroll

@@ -57,12 +57,23 @@ def train_main(argv):
     raise ValueError(f'WORLD_SIZE={st.world_size} but --distribute is not set: launch one process, or pass --distribute '
                      'for data-parallel training.')
   input_fn = synthetic.train_input_fn
+  weak = [f for f in ('per_bbox_split_path', 'per_image_split_path') if getattr(st, f)]
+  if weak and not st.per_pixel_split_path and not st.synthetic:
+    raise ValueError(f'--{weak[0]} needs --per_pixel_split_path: the weak parts of the batch are trained with per-pixel '
+                     'examples (training on weak labels alone is not supported).')
   if st.per_pixel_split_path and not st.synthetic:
     from wlseg import train_input
     pairs = train_input.split_pairs(st.per_pixel_split_path, st.per_pixel_dataset_name)
+    if weak:
+      parts = ('the bounding-box part from --per_bbox_split_path' if st.per_bbox_split_path else
+               'the bounding-box part empty (no --per_bbox_split_path)',
+               'the image-level part from --per_image_split_path' if st.per_image_split_path else
+               'the image-level part empty (no --per_image_split_path)')
+      weak_note = f'{parts[0]}, {parts[1]}.'
+    else:
+      weak_note = 'the bounding-box and image-level parts of the batch are empty (there is no Open Images source).'
     print(f'Training on the {st.per_pixel_dataset_name} split at {st.per_pixel_split_path}: {len(pairs)} image / label '
-          f'pairs, {len(pairs[st.rank::st.world_size])} on this rank; the bounding-box and image-level parts of the batch '
-          'are empty (there is no Open Images source).', flush=True)
+          f'pairs, {len(pairs[st.rank::st.world_size])} on this rank; {weak_note}', flush=True)
     input_fn = train_input.train_input_fn
   system = SemanticSegmentation({'train': input_fn}, None, st)
   out = system.train()

@@ -23,6 +23,14 @@ WEAK_CLASSES = ('bicycle', 'bus', 'car', 'motorcycle', 'train', 'truck',
                 'human', 'man', 'woman', 'boy', 'girl',
                 'traffic light', 'traffic sign', 'stop sign', 'void')
 WEAK_HUMANS = ('human', 'man', 'woman', 'boy', 'girl')
+# Open Images display names (class-descriptions-boxable.csv) of the weak classes whose name here differs
+WEAK_DISPLAY_NAMES = {'human': 'Person'}
+
+
+def weak_display_name(cid):
+  """Open Images display name of weak class `cid` (compared case-insensitively)."""
+  name = WEAK_CLASSES[cid]
+  return WEAK_DISPLAY_NAMES.get(name, name[0].upper() + name[1:])
 
 _DATASETS = {
     'cityscapes': dict(

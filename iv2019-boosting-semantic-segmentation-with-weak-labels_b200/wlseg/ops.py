@@ -113,6 +113,8 @@ _SIGNATURES = {
                                          _vp, _vp, _vp]),
     'wlseg_train_inputs': (ctypes.c_int, [_vp, _vp, _vp, _c_int, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp,
                                           _vp, _vp]),
+    'wlseg_weak_train_inputs': (ctypes.c_int, [_vp, _vp, _vp, _vp, _c_int, _vp, _vp, _vp, _vp, _vp, _vp, _c_int, _c_int,
+                                               _c_int, _vp, _vp, _vp, _vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
@@ -672,3 +674,38 @@ def train_inputs(arena, offsets, sizes, index, lut, void_id, target_hw, proimage
          'wlseg_train_inputs')
   _count()
   return proimages, prolabels
+
+
+def weak_train_inputs(arena, offsets, sizes, resized, index, crops, target_hw, proimages, labels, invalid, boxes=None,
+                      vectors=None):
+  """Arena images selected by a device index vector and cut at per-output crop offsets -> one weak part of the training
+  contract, one launch (wlseg_weak_train_inputs).  arena uint8 [bytes] (example e: RGB HWC at offsets[e]), offsets int64
+  [E], sizes / resized int32 [E, 2] = (H, W) / the aspect-preserving resized size, index int32 [N], crops int32 [N, 2] =
+  (oy, ox).  Exactly one of boxes = (box_start int32 [E + 1], box_coords fp32 [B, 4] = xmin, xmax, ymin, ymax,
+  box_cids int32 [B]) for the bounding-box part and vectors fp32 [E, 15] for the image-level part.  Writes proimages
+  fp32 [N, TH, TW, 3] and labels fp32 [N, TH, TW, 15]; invalid (int64 [1]) += the out-of-range indices and crops."""
+  N, E = index.numel(), offsets.numel()
+  TH, TW = int(target_hw[0]), int(target_hw[1])
+  assert (boxes is None) != (vectors is None), 'one of boxes (bounding-box part) and vectors (image-level part)'
+  assert arena.dtype == torch.uint8 and arena.dim() == 1 and arena.is_contiguous()
+  assert offsets.dtype == torch.int64 and offsets.is_contiguous() and offsets.dim() == 1
+  for t in (sizes, resized):
+    assert t.dtype == torch.int32 and t.is_contiguous() and tuple(t.shape) == (E, 2)
+  assert index.dtype == torch.int32 and index.is_contiguous() and index.dim() == 1
+  assert crops.dtype == torch.int32 and crops.is_contiguous() and tuple(crops.shape) == (N, 2)
+  assert proimages.dtype == torch.float32 and proimages.is_contiguous() and tuple(proimages.shape) == (N, TH, TW, 3)
+  assert labels.dtype == torch.float32 and labels.is_contiguous() and tuple(labels.shape) == (N, TH, TW, 15)
+  assert invalid.dtype == torch.int64
+  start = coords = cids = None
+  if boxes is not None:
+    start, coords, cids = boxes
+    assert start.dtype == torch.int32 and start.is_contiguous() and tuple(start.shape) == (E + 1,)
+    assert coords.dtype == torch.float32 and coords.is_contiguous() and coords.dim() == 2 and coords.shape[1] == 4
+    assert cids.dtype == torch.int32 and cids.is_contiguous() and tuple(cids.shape) == (coords.shape[0],)
+  else:
+    assert vectors.dtype == torch.float32 and vectors.is_contiguous() and tuple(vectors.shape) == (E, 15)
+  _check(lib().wlseg_weak_train_inputs(_ptr(arena), _ptr(offsets), _ptr(sizes), _ptr(resized), E, _ptr(start),
+                                       _ptr(coords), _ptr(cids), _ptr(vectors), _ptr(index), _ptr(crops), N, TH, TW,
+                                       _ptr(proimages), _ptr(labels), _ptr(invalid), _stream()), 'wlseg_weak_train_inputs')
+  _count()
+  return proimages, labels

@@ -8,7 +8,7 @@ flags (code/predict.py:171-197) and the per-script hard overrides (`_add_extra_a
 code/train.py:42-68, code/evaluate.py:69-79, code/predict.py:199-211).
 
 Additive flags of this implementation (absent upstream): --synthetic, --dtype, --steps, --seed, and for train.py
---per_pixel_split_path.
+--per_pixel_split_path, --per_bbox_split_path and --per_image_split_path.
 """
 
 import argparse
@@ -63,6 +63,14 @@ class SemanticSegmentationArguments(object):
       p.add_argument('--per_pixel_split_path', type=str, default=None, metavar='DIR',
                      help='Training split of the per-pixel dataset (a Cityscapes leftImg8bit/<split> directory or a Vistas '
                           'split directory with images/ + labels/), decoded once into device memory.')
+      p.add_argument('--per_bbox_split_path', type=str, default=None, metavar='DIR',
+                     help='Open Images directory (class-descriptions-boxable.csv, one *annotations-bbox.csv, '
+                          'images/<ImageID>.jpg) of the bounding-box part of the batch, decoded once into device memory. '
+                          'Needs --per_pixel_split_path; may name the same directory as --per_image_split_path.')
+      p.add_argument('--per_image_split_path', type=str, default=None, metavar='DIR',
+                     help='Open Images directory (class-descriptions-boxable.csv, one '
+                          '*annotations-human-imagelabels*.csv, images/<ImageID>.jpg) of the image-level part of the '
+                          'batch, decoded once into device memory.  Needs --per_pixel_split_path.')
 
   def add_train_arguments(self):
     p = self._parser

@@ -10,8 +10,8 @@ launch (ops.train_inputs) over a device-resident permutation.
 Files are found and checked by wlseg.dataset_input (the layouts its docstring lists).  Rank r of R owns the files i with
 i % R == r.  Each epoch is a fresh permutation of the rank's shard, a pure function of (seed, rank, world, epoch); every
 rank takes the same number of batches per epoch and drops the rest, so a run resumed at global step k feeds exactly the
-batches an uninterrupted run feeds from step k on.  The batch carries the per-pixel part only: there is no Open Images
-source for the bounding-box and image-level parts.
+batches an uninterrupted run feeds from step k on.  The bounding-box and image-level parts of the batch come from Open
+Images splits (wlseg.weak_input) when train.py names them, and are empty otherwise.
 """
 
 import time
@@ -28,6 +28,11 @@ from wlseg.dataset_input import DatasetError
 # Estimator.train after the network exists: 10.37 GB at Cityscapes 4 x 512 x 1024, 10.94 GB at Vistas 4 x 621 x 855.
 # The reserve is the larger of the two plus a quarter, rounded up to whole GiB.
 STEP_RESERVE_BYTES = 13 << 30
+# The same for the mixed 4 + 8 + 4 step (per-pixel + bounding-box + image-level examples), which holds four times the
+# images of a per-pixel-only step and its 15-way dense weak labels.  NOT MEASURED yet: an estimate, the Vistas
+# per-pixel footprint above scaled to 16 images (4 x 10.94 GB = 43.76 GB) plus a quarter (54.7 GB), rounded up to 51
+# GiB.  tools/weak_dataset_bench.py measures it (mixed_step_footprint_bytes, DESIGN.md 8.3).
+MIXED_STEP_RESERVE_BYTES = 51 << 30
 
 
 def split_pairs(path, dataset_name):
@@ -44,10 +49,12 @@ def steps_per_epoch(n_files, world, Nb):
   return (n_files // world) // Nb
 
 
-def epoch_order(seed, rank, world, n_files, Nb, epoch):
-  """Shard positions rank `rank` feeds in epoch `epoch`, in order: a permutation of its shard cut to whole batches."""
+def epoch_order(seed, rank, world, n_files, Nb, epoch, rng=None):
+  """Shard positions rank `rank` feeds in epoch `epoch`, in order: a permutation of its shard cut to whole batches.
+  `rng` replaces the per-pixel generator of (seed, rank, world, epoch) (the weak parts draw from their own)."""
   n_shard = len(range(rank, n_files, world))
-  rng = np.random.default_rng([seed % (1 << 64), rank, world, epoch])
+  if rng is None:
+    rng = np.random.default_rng([seed % (1 << 64), rank, world, epoch])
   return rng.permutation(n_shard)[:steps_per_epoch(n_files, world, Nb) * Nb].astype(np.int32)
 
 
@@ -57,21 +64,29 @@ def batch_at(seed, rank, world, n_files, Nb, global_step):
   return epoch_order(seed, rank, world, n_files, Nb, epoch)[k * Nb:(k + 1) * Nb]
 
 
-def arena_layout(sizes):
-  """-> (int64 byte offsets of the examples, total bytes): each holds H * W * 3 image bytes, then H * W label ids."""
-  nbytes = np.asarray([h * w * 4 for h, w in sizes], dtype=np.int64)
+def arena_layout(sizes, bytes_per_pixel=4):
+  """-> (int64 byte offsets of the examples, total bytes): each holds H * W * 3 image bytes, then (4 bytes per pixel,
+  per-pixel examples) H * W label ids."""
+  nbytes = np.asarray([h * w * bytes_per_pixel for h, w in sizes], dtype=np.int64)
   offsets = np.zeros(len(sizes), dtype=np.int64)
   np.cumsum(nbytes[:-1], out=offsets[1:])
   return offsets, int(nbytes.sum())
 
 
-def device_budget(device):
-  """Arena bytes the device can hold next to a training step (None on the CPU: no limit)."""
+def device_budget(device, reserve=STEP_RESERVE_BYTES):
+  """Arena bytes the device can hold next to a training step that needs `reserve` bytes (None on the CPU: no limit)."""
   device = torch.device(device)
   if device.type != 'cuda':
     return None
   free, _ = torch.cuda.mem_get_info(device)
-  return free - STEP_RESERVE_BYTES
+  return free - reserve
+
+
+def check_budget(what, need, budget):
+  """Refuses `need` bytes of decoded examples over `budget` (None: no limit), naming `what`."""
+  if budget is not None and need > budget:
+    raise DatasetError(f'{what} needs {need} bytes of device memory but {max(budget, 0)} are available next to a '
+                       'training step; more ranks (--distribute) shrink each shard')
 
 
 class _Examples(torch.utils.data.Dataset):
@@ -103,17 +118,18 @@ class _Examples(torch.utils.data.Dataset):
 class Shard:
   """One rank's examples in one uint8 arena on `device`: .arena, .offsets (int64 [E]), .sizes (int32 [E, 2])."""
 
-  def __init__(self, pairs, sizes, n_lids, device, budget=None, workers=None):
-    """Checks the arena against `budget` bytes (None: no limit) before anything is decoded, then fills it."""
+  def __init__(self, pairs, sizes, n_lids, device, budget=None, workers=None, examples=None, bytes_per_pixel=4):
+    """Checks the arena against `budget` bytes (None: no limit) before anything is decoded, then fills it.  `examples`
+    (default: the per-pixel image / label pairs) is a dataset of (i, uint8 [H * W * bytes_per_pixel]) items."""
     device = torch.device(device)
-    offsets, total = arena_layout(sizes)
-    if budget is not None and total > budget:
-      raise DatasetError(f'the decoded shard of {len(pairs)} files needs {total} bytes of device memory but {max(budget, 0)} '
-                         'are available next to a training step; more ranks (--distribute) shrink each shard')
+    offsets, total = arena_layout(sizes, bytes_per_pixel)
+    check_budget(f'the decoded shard of {len(pairs)} files', total, budget)
     t0 = time.perf_counter()
     self.arena = torch.empty(total, dtype=torch.uint8, device=device)
     workers = min(workers or dataset_input._workers_per_rank(), len(pairs))
-    loader = torch.utils.data.DataLoader(_Examples(pairs, sizes, n_lids), batch_size=None, shuffle=False,
+    if examples is None:
+      examples = _Examples(pairs, sizes, n_lids)
+    loader = torch.utils.data.DataLoader(examples, batch_size=None, shuffle=False,
                                          num_workers=workers, pin_memory=device.type == 'cuda')
     for i, chunk in loader:
       off = int(offsets[i])
@@ -147,16 +163,32 @@ def train_input_fn(config, params):
           'training on the files found.', flush=True)
   mine = pairs[rank::world]
   sizes, _, _ = dataset_input.check_pairs(mine)
+  hw = (params.height_feature_extractor, params.width_feature_extractor)
+  from wlseg import weak_input
+  weak = weak_input.parts(params, hw, rank, world)   # CSVs and headers only: nothing is decoded yet
+  for part in weak:
+    print(f'{"" if world == 1 else f"rank {rank}: "}{part.summary()}', flush=True)
+  budget = None
+  if weak:
+    check_budget('the decoded per-pixel, bounding-box and image-level shards', arena_layout(sizes)[1] +
+                 sum(part.bytes for part in weak), device_budget(device, MIXED_STEP_RESERVE_BYTES))
+  else:
+    budget = device_budget(device)
   table = _replacevoids(params.training_problem_def['lids2cids'])
-  shard = Shard(mine, sizes, len(table), device, budget=device_budget(device))
+  shard = Shard(mine, sizes, len(table), device, budget=budget)
   print(f'{"" if world == 1 else f"rank {rank}: "}decoded {shard.files} files into {shard.bytes} bytes of '
         f'{device.type} memory in {shard.seconds:.1f} s', flush=True)
+  for part in weak:
+    part.fill(device)
   lut = torch.tensor(table, dtype=torch.int32, device=device)
-  hw = (params.height_feature_extractor, params.width_feature_extractor)
   n, spe, step = len(pairs), steps_per_epoch(len(pairs), world, Nb), int(getattr(params, 'initial_global_step', 0))
-  # two output pairs: the estimator's prefetcher enqueues batch i + 1 before step i copies batch i into its inputs
-  ring = [(torch.empty((Nb,) + hw + (3,), dtype=torch.float32, device=device),
-           torch.empty((Nb,) + hw, dtype=torch.int32, device=device)) for _ in range(2)]
+  rows = Nb + sum(part.Nb for part in weak)
+  # two output sets: the estimator's prefetcher enqueues batch i + 1 before step i copies batch i into its inputs.
+  # proimages holds the per-pixel rows, then the bounding-box rows, then the image-level rows.
+  ring = [(torch.empty((rows,) + hw + (3,), dtype=torch.float32, device=device),
+           torch.empty((Nb,) + hw, dtype=torch.int32, device=device),
+           [torch.empty((part.Nb,) + hw + (15,), dtype=torch.float32, device=device) for part in weak])
+          for _ in range(2)]
   invalid = torch.zeros(1, dtype=torch.int64, device=device)
 
   def batches(step):
@@ -167,9 +199,15 @@ def train_input_fn(config, params):
         if int(invalid.item()):
           raise ops.WlsegError(f'{int(invalid.item())} label ids or indices outside the training arena\'s tables')
         order = torch.from_numpy(epoch_order(params.seed, rank, world, n, Nb, epoch)).to(device)
-      pro, lab = ring[step % 2]
-      ops.train_inputs(shard.arena, shard.offsets, shard.sizes, order[k * Nb:(k + 1) * Nb], lut, max(table), hw, pro, lab,
-                       invalid)
-      yield {'proimages': pro}, {'prolabels_per_pixel': lab}
+      pro, lab, weak_labels = ring[step % 2]
+      ops.train_inputs(shard.arena, shard.offsets, shard.sizes, order[k * Nb:(k + 1) * Nb], lut, max(table), hw, pro[:Nb],
+                       lab, invalid)
+      labels = {'prolabels_per_pixel': lab}
+      row = Nb
+      for part, out in zip(weak, weak_labels):
+        part.gather(step, pro[row:row + part.Nb], out)
+        labels[part.label_key] = out
+        row += part.Nb
+      yield {'proimages': pro}, labels
       step += 1
   return batches(step)
